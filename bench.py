@@ -30,12 +30,15 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tools"))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from as it found it
 
 GENOME_MB = float(os.environ.get("HB_BENCH_GENOME_MB", "100"))
 REF_SAMPLE_MB = float(os.environ.get("HB_BENCH_REF_MB", "4"))
 COV = float(os.environ.get("HB_BENCH_COV", "30"))
 SEED = 20260923
 METRIC = "HiFi Gbp overlapped/sec"
+DUMP_READS = 128              # --dump-outputs: reads whose overlap records and corrected bases are written
+DUMP_PER_READ_MAX = 800000    # --dump-outputs: reads whose per-read values are written (every read of a set up to this size)
 
 
 def workload_name(mb):
@@ -137,6 +140,37 @@ def algorithmic_bytes(kernel, c, bases):
     return float(f.get(kernel, 0))
 
 
+def dump_outputs(d, eng, r):
+    """What the last timed step computed, as d/<name>.npy (float64; 0/1 flags and bases float32), at most 64 MB in all so that two builds can be compared
+    output for output: per-read values of every read (of a seeded sample above DUMP_PER_READ_MAX reads) — the overlap counts of both final lists, the two
+    read flags, the corrected lengths — and, for a seeded sample of DUMP_READS reads, every field of their final overlap records and their corrected
+    bases (0-3, 4 = N); the coverage peaks and corrected bases per round in stage_scalars."""
+    n = eng.n_reads
+    rng = np.random.default_rng(SEED)
+    per = np.arange(n) if n <= DUMP_PER_READ_MAX else np.sort(rng.choice(n, DUMP_PER_READ_MAX, replace=False))
+    pick = np.sort(rng.choice(n, min(n, DUMP_READS), replace=False))
+    rs = eng.download_reads()
+    out = {"per_read_ids": per, "sample_read_ids": pick, "stage_scalars": np.array([r["hom_cov"], r["het_cov"]] + r["corrected_bases"]),
+           "corrected_length": rs.length[per], "is_fully_corrected": r["is_fully_corrected"][per].astype(np.float32),
+           "is_abnormal": r["is_abnormal"][per].astype(np.float32),
+           "sample_corrected_bases": np.concatenate([rs.decode(int(i)) for i in pick]).astype(np.float32)}
+    for lst in ("src", "rev"):
+        off = r[lst + "_off"].astype(np.int64)
+        out[lst + "_per_read"] = np.diff(off)[per]
+        rec = np.concatenate([r[lst][off[i]:off[i + 1]] for i in pick])
+        # columns: qn, qs (the two halves of qns), qe, tn, ts, te, ml, rev, bl, del, el, no_l_indel
+        out["sample_" + lst + "_records"] = np.stack([rec["qns"] >> np.uint64(32), rec["qns"] & np.uint64(0xffffffff)] +
+                                                     [rec[f] for f in ("qe", "tn", "ts", "te", "ml", "rev", "bl", "del", "el", "no_l_indel")], axis=1)
+    out = {k: (a if a.dtype == np.float32 else a.astype(np.float64)) for k, a in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    if total > 64 << 20:
+        raise RuntimeError("--dump-outputs: %d bytes would exceed 64 MB" % total)
+    os.makedirs(d, exist_ok=True)
+    for k, a in out.items():
+        np.save(os.path.join(d, k + ".npy"), a)
+    return total
+
+
 _JSON_OUT = None
 
 
@@ -165,7 +199,12 @@ def _main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this project's stage computed; the reference binary keeps its own files")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     threads = len(os.sched_getaffinity(0))
     dtype = "u8/u64/f64 (2-bit bases, 64-bit bit-vectors, double chain scores)"
@@ -251,6 +290,9 @@ def _main():
                 a = kms.setdefault(k, [0, 0.0]); a[0] += v[0]; a[1] += v[1]
             last_ms = r["ms"]
     barrier()
+    if args.dump_outputs and rank == 0:
+        nb = dump_outputs(args.dump_outputs, eng, r)
+        sys.stderr.write("[bench] outputs of the last timed step: %d bytes in %s\n" % (nb, args.dump_outputs))
     clocks = cs.summary()
     dev_ms_max, _ = hdist.reduce_time_and_units(dev_ms, 0.0, device="cuda")
     e2e_max, _ = hdist.reduce_time_and_units(e2e_s, 0.0, device="cuda")

@@ -192,7 +192,9 @@ HB_HD uint64_t hb_cns_push0(CnsCtx &C, uint32_t len0, uint32_t rc, int64_t qoff)
 	return nec;
 }
 
-HB_HD uint64_t hb_cns_full_(CnsCtx &C, int64_t s0, int64_t e0); // cns_gen_full (hb_eccns_full.cuh); sets C.need_full = 2 when the arena is too small
+// cns_gen_full (hb_eccns_full.cuh); sets C.need_full = 2 when the arena is too small.  Out of line: inlined into k_ec_cns_w<true>, the one kernel
+// that calls it, the graph code kept cicc (CUDA 12.9) busy for a quarter of an hour; as a call it compiles in seconds.
+HB_HD_NI uint64_t hb_cns_full_(CnsCtx &C, int64_t s0, int64_t e0);
 // push_cns_anchor, ecovlp.cpp:2109-2163
 template <bool GRAPH> HB_HD uint64_t hb_cns_anchor(CnsCtx &C, uint64_t s, uint64_t e, int is_tail)
 {

@@ -524,7 +524,7 @@ HB_HD uint64_t hb_cns_full(CnsCtx &C, CnsG &G, int64_t s0, int64_t e0)
 	for (; s < e0 && !G.ovf;) { nec += hb_cns_full0(C, G, s, e, s == s0 ? 1 : 0); s += HB_CNS_G_WL; e += HB_CNS_G_WL; if (e > e0) e = e0; }
 	return nec;
 }
-HB_HD uint64_t hb_cns_full_(CnsCtx &C, int64_t s0, int64_t e0)
+HB_HD_NI uint64_t hb_cns_full_(CnsCtx &C, int64_t s0, int64_t e0)
 {
 	const uint64_t nec = hb_cns_full(C, *C.g, s0, e0);
 	if (C.g->ovf) C.need_full = 2;

@@ -49,6 +49,40 @@ class Golden:
         return self.z["%s_n_%s" % (mode, stage)]
 
 
+STAGE_FILES = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "stage_files.npz")
+
+
+def stage_file_digests(prefix):
+    """{file suffix: (size, blake2b-128 hex)} of the files a whole stage writes under `prefix` (-o prefix --write-paf --write-ec).
+    .ec.bin is taken by what it holds (lengths, reads with the pad bytes the reference leaves undefined masked, names, coverage peaks), its size by
+    the number of reads."""
+    out = {}
+    for suf in ("ovlp.paf", "ec.fa", "ovlp.source.bin", "ovlp.reverse.bin"):
+        b = open(prefix + "." + suf, "rb").read()
+        out[suf] = (len(b), hashlib.blake2b(b, digest_size=16).hexdigest())
+    rs = binio.load_ec_bin(prefix + ".ec.bin")
+    h = hashlib.blake2b(digest_size=16)
+    for part in (rs.length.astype("<u8").tobytes(), binio.canonical_packed(rs).tobytes(), rs.name_blob, np.array([rs.hom_cov, rs.het_cov], "<i4").tobytes()):
+        h.update(part)
+    out["ec.bin"] = (rs.n, h.hexdigest())
+    return out
+
+
+def diff_digests(want, got):
+    """the files whose digests differ, with both (size, digest) pairs"""
+    return ["%s (%s vs %s)" % (k, want[k], got.get(k)) for k in sorted(want) if want[k] != got.get(k)]
+
+
+def stored_stage_digests(genome_mb, cov, seed, n_rate):
+    """stage_file_digests of the unmodified reference binary's files for the tools/simgen.py read set of these parameters
+    (tests/golden/stage_files.npz, made by tests/golden/make_stage_files.py); None when that set is not stored"""
+    z = np.load(STAGE_FILES)
+    for name in str(z["sets"]).split(","):
+        if tuple(z[name + "_params"]) == (float(genome_mb), float(cov), float(seed), float(n_rate)):
+            return {str(s): (int(n), str(d)) for s, n, d in zip(z[name + "_suffix"], z[name + "_size"], z[name + "_dg"])}
+    return None
+
+
 def chain_digest(ch, fc_pool):
     """digest of chain records + fake cigars, the way make_golden.read_stages does.
     ch: structured array with fields of CH plus fc_off/fc_n"""
